@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """bench.py — headline measurement of the PLONK-prover hot path (DESIGN.md §6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log-gates L]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log-gates L] [--dump-outputs DIR]
+
+--steps K is the number of timed steps of the headline and of the MSM, NTT and large-prove context objects.
+--dump-outputs DIR writes the proof of the last timed step to DIR/proof.npy; the inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 
 Headline (BASELINE.json `metric`, first item; configs[3]): **PLONK prove time at 2^20 gates** — one step = one proof
 of the synthetic arithmetic circuit (mul / add chain, boolean padding, 2 public inputs; SURVEY.md §8d): 11 G1 MSMs of
@@ -36,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the checkout may be read-only: leave no __pycache__ in it
 
 R_MOD = 0x73EDA753299D7D483339D80809A1D80553BDA402FFFE5BFEFFFFFFFF00000001
 FR_MONT_R = (1 << 256) % R_MOD
@@ -144,6 +149,13 @@ def headline_metric(L):
     return "PLONK prove time (BLS12-381 / KZG10, synthetic arithmetic circuit, 2^%d gates)" % L
 
 
+def dump_outputs(out_dir, proof):
+    """The 1040 proof bytes (11 compressed G1 commitments, then 16 scalar evaluations) as float64, which holds every
+    byte value exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "proof.npy"), np.frombuffer(proof, dtype=np.uint8).astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------- clocks
 class ClockSampler:
     FIELDS = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
@@ -214,6 +226,8 @@ def run_reference(args, rank, world):
     while sample_log > 12 and (cal_pre + args.steps * cal_prove) * scale * 2.0 ** (sample_log - L) > budget - (time.perf_counter() - t_start):
         sample_log -= 1
     proof, _, t_pre, t_steps = cpu_prove(sample_log, cores, reps=args.steps)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof)
     ms = 1e3 * sum(t_steps) / len(t_steps)
     same = sample_log == L
     sample = ("each step = one full prove_with_preprocessed of the SAME 2^%d-gate circuit (C restatement of dusk-plonk 0.8, oracle/plonk_oracle.inc), "
@@ -313,7 +327,8 @@ def timed_proves(setup, args, torch, stream, dist=None, device=None):
     torch.cuda.cudart().cudaProfilerStart()   # `ncu --profile-from-start off` then lists exactly the launches of the timed steps
     e0.record(stream)
     for _ in range(args.steps):
-        proofs.add(setup.prove_dev())
+        last_proof = setup.prove_dev()
+        proofs.add(last_proof)
     e1.record(stream)
     barrier()
     torch.cuda.cudart().cudaProfilerStop()
@@ -342,7 +357,7 @@ def timed_proves(setup, args, torch, stream, dist=None, device=None):
         dev_ms, e2e_ms, wall_dev_ms = v[:3]
         rounds = {"round%d" % k: v[2 + k] for k in range(1, 6)}
     return {"dev_ms": dev_ms, "e2e_ms": e2e_ms, "wall_dev_ms": wall_dev_ms, "proofs": proofs, "launches": int(launches), "clocks": clocks,
-            "sums": sums, "rounds_ms": {k: round(v, 3) for k, v in rounds.items()}}
+            "sums": sums, "rounds_ms": {k: round(v, 3) for k, v in rounds.items()}, "last_proof": last_proof}
 
 
 def prove_roofline(setup, timed, args, imad_peak, n_per_msm):
@@ -391,6 +406,8 @@ def run_ours(args, rank, world, local_rank):
         ctx.comm_init_from_torch(dist)   # torch.distributed only carries the 128-byte NCCL id
     setup = ProveSetup(ctx, L, torch, shard=(rank, world) if world > 1 else None, dist=dist, device=device, lib_collectives=lib_coll)
     timed = timed_proves(setup, args, torch, stream, dist, device)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, timed["last_proof"])
     proof = next(iter(timed["proofs"]))
     parity = {"deterministic": len(timed["proofs"]) == 1, "verifier_accepts": bool(setup.verify(proof)) if rank == 0 else None}
     extra = {}
@@ -537,7 +554,7 @@ def bench_msm(ctx, stream, args, torch, imad_peak, dist, rank, world, device):
     msm_scalar_slice(LT, rank, world, s_host)
     s_dev = ctx.malloc(n * 32)
     ctx.h2d(s_dev, s_host)
-    steps = max(3, min(args.steps, 5))
+    steps = args.steps
 
     def barrier():
         if dist is not None:
@@ -652,7 +669,7 @@ def bench_ntt_sharded(ctx, dist, rank, world, args, torch):
         dom.fft(buf, tmp)
     dist.barrier(); ctx.sync(); torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(args.steps, 10)
+    reps = args.steps
     e0.record(be.stream)
     for _ in range(reps):
         dom.fft(buf, tmp)
@@ -732,7 +749,7 @@ def bench_ntt(ctx, stream, args, imad_peak, torch):
         ctx.ntt_dev(d, L, 0, 0)
     ctx.sync()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    reps = max(args.steps, 10)
+    reps = args.steps
     l0 = ctx.launch_count()
     e0.record(stream)
     for _ in range(reps):
@@ -789,7 +806,7 @@ def bench_prove_large(ctx, args, torch, stream, dist=None, rank=0, world=1, devi
     L = args.large_log_gates
     s = ProveSetup(ctx, L, torch, shard=(rank, world) if world > 1 else None, dist=dist, device=device, lib_collectives=args.collectives == "lib")
     proofs = {s.prove_host() for _ in range(2)}
-    reps = 3
+    reps = args.steps
     ctx.profile_enable(True)
     ctx.profile_reset()
     t = []
@@ -852,7 +869,10 @@ def main():
     ap.add_argument("--skip-single-check", action="store_true", help="N > 1: skip rank 0's single-GPU 2^24 proof")
     ap.add_argument("--collectives", default="lib", choices=["lib", "torch"],
                     help="N > 1: NCCL inside the library (pb200_comm) or torch.distributed callbacks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step to DIR/proof.npy (float64 bytes)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,5 +1,6 @@
 """CPU tests of bench.py's host logic: the reference arm runs the checker only (it must never load the product
 library), reports the circuit it actually proved, and the checker's circuit generator is the product's, row for row."""
+import hashlib
 import json
 import os
 import subprocess
@@ -24,12 +25,12 @@ def test_oracle_synthetic_circuit_equals_product_helpers(oracle):
             assert (a[2] == b[2]).all() and (a[3] == b[3]).all() and (a[4] == b[4]).all()
 
 
-def test_reference_arm_runs_without_the_product_library():
+def test_reference_arm_runs_without_the_product_library(tmp_path):
     code = ("import sys, runpy\n"
-            "sys.argv = ['bench.py', '--impl', 'reference', '--log-gates', '10', '--steps', '2', '--warmup', '1']\n"
+            "sys.argv = ['bench.py', '--impl', 'reference', '--log-gates', '10', '--steps', '2', '--warmup', '1', '--dump-outputs', %r]\n"
             "runpy.run_path(%r, run_name='__main__')\n"
             "assert not any(m.startswith('plonk_prototype_b200') for m in sys.modules), 'product package imported'\n"
-            "assert 'libpb200' not in open('/proc/self/maps').read(), 'product library mapped'\n" % os.path.join(ROOT, "bench.py"))
+            "assert 'libpb200' not in open('/proc/self/maps').read(), 'product library mapped'\n" % (str(tmp_path), os.path.join(ROOT, "bench.py")))
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd=ROOT, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     line = json.loads(r.stdout.strip().splitlines()[-1])
@@ -37,6 +38,9 @@ def test_reference_arm_runs_without_the_product_library():
     assert line["steps"] == 2 and len(line["steps_ms"]) == 2 and line["same_config"] is True
     assert line["config"]["log_gates"] == 10 and line["sample_log_gates"] == 10
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+    proof = np.load(tmp_path / "proof.npy")
+    assert proof.dtype == np.float64 and proof.shape == (1040,)
+    assert hashlib.sha256(proof.astype(np.uint8).tobytes()).hexdigest()[:16] == line["proof_sha256_16"]
 
 
 def test_reference_arm_bounds_its_sample_and_says_so():
