@@ -16,8 +16,9 @@
 //     kernel bound by dispatch slots; the last pass stores canonical values;
 //   * the bit reversal and the inter-pass twiddle / coset factor are applied in registers after the last round, the
 //     results go to shared memory at their output row, and one elected thread issues the tensor store.
-// Used for transforms of 2^12 … 2^27 points (two passes up to 2^18, three above; S ∈ 6…9); everything else, and the
-// peer-store variant of the sharded transform, stays on ntt_pass_kernel.
+// Used for transforms of 2^12 … 2^26 points (two passes up to 2^18, three above; S ∈ 6…9) whose plan has single-lookup tables;
+// everything else (2^27 and up, plans built after the table budget ran out), and the peer-store variant of the sharded
+// transform, stays on ntt_pass_kernel.
 #pragma once
 // (ntt.cu includes <cuda.h> and defines Fr, g_load, g_store, bfly, bfly1 before including this file inside its namespace)
 
