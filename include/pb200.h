@@ -151,6 +151,27 @@ PB200_API int pb200_srs_generate(pb200_ctx *ctx, const uint64_t tau_mont[4], siz
 PB200_API int pb200_srs_generate_range(pb200_ctx *ctx, const uint64_t tau_mont[4], size_t first, size_t n_points, pb200_srs **out);
 /* Device address of an SRS's packed affine points (n × 96 B), e.g. to serialise the CommitKey. */
 PB200_API const uint64_t *pb200_srs_dev_ptr(const pb200_srs *srs);
+/* Per-point result of G1Affine::from_bytes on a 48-byte compressed (zcash) encoding. */
+enum {
+    PB200_G1_OK = 0,
+    PB200_G1_BAD_FLAGS = 1,       /* bit 7 clear, or bit 6 (identity) set on anything but c0 00…00 */
+    PB200_G1_X_RANGE = 2,         /* x ≥ p */
+    PB200_G1_NOT_ON_CURVE = 3,    /* x³ + 4 is not a square */
+    PB200_G1_NOT_IN_SUBGROUP = 4, /* on the curve, outside the prime-order subgroup */
+    PB200_G1_IDENTITY = 5         /* the canonical identity encoding: valid upstream, not representable here */
+};
+/* CommitKey::from_slice over a whole key (G1Affine::from_bytes per point): n_points 48-byte compressed encodings on the HOST
+ * are decoded and checked on the device (flags, x < p, on the curve, prime-order subgroup) and kept resident as an SRS in the
+ * layout of pb200_srs_upload.  Any invalid point: PB200_ERR_ARG, pb200_last_error names the first invalid index and its
+ * reason, *out is left untouched and nothing stays allocated.  status_host (optional, n_points bytes): PB200_G1_* per point.
+ * The identity encoding is rejected (PB200_G1_IDENTITY): the ABI cannot hold it and a commit key never contains it.
+ * 1 ≤ n_points < 2^31.  A rank of a point-range-sharded prover loads its slice powers_of_g[first .. first + n) by passing
+ * bytes_host + 48·first and n: the encoding has no prefix, so no other entry point is needed.  Blocks. */
+PB200_API int pb200_srs_from_compressed(pb200_ctx *ctx, const uint8_t *bytes_host, size_t n_points, uint8_t *status_host,
+                                        pb200_srs **out);
+/* CommitKey::to_var_bytes: points [offset, offset + n) of an SRS as 48-byte compressed encodings, 48·n bytes on the HOST.
+ * 1 ≤ n < 2^31 and the range must lie inside the SRS.  Blocks. */
+PB200_API int pb200_srs_to_compressed(pb200_ctx *ctx, const pb200_srs *srs, size_t offset, size_t n, uint8_t *bytes_host);
 /* CommitKey::compute_single_witness: p(z) and q(X) = (p(X) − p(z)) / (X − z) for a device-resident polynomial of
  * n coefficients (Ruffini's rule as scale → Fr suffix scan → scale).  quotient_dev receives n scalars (the top one
  * is zero).  Blocks; p(z) is returned on the host. */
@@ -283,7 +304,8 @@ PB200_API int pb200_synthetic_circuit(size_t n_gates, uint64_t seed, uint32_t n_
                                       uint64_t *values_mont, size_t n_vars_capacity, size_t *n_vars_out, uint32_t *pi_gate,
                                       uint64_t *pi_mont);
 /* Per-kernel device time of the most recent MSM / NTT call, from CUDA events on the context stream.
- * Known names: "msm.accumulate", "msm.sort", "msm.reduce", "msm.total", "ntt.total".
+ * Known names: "msm.accumulate", "msm.sort", "msm.reduce", "msm.total", "ntt.total", and "srs.decompress" / "srs.compress"
+ * (the kernels of pb200_srs_from_compressed / pb200_srs_to_compressed).
  * Profiling must have been switched on before that call. */
 PB200_API int pb200_profile_enable(pb200_ctx *ctx, int on);
 PB200_API int pb200_profile_ms(pb200_ctx *ctx, const char *name, float *ms);

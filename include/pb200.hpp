@@ -213,6 +213,24 @@ class CommitKey {
         if (max_degree + 1 <= ((size_t)1 << 22)) ctx.check(pb200_srs_precompute(ctx.raw(), srs), "pb200_srs_precompute");
         return CommitKey(ctx, srs);
     }
+    // CommitKey::from_slice: 48-byte compressed points, each decoded and checked on the device like G1Affine::from_bytes (flags,
+    // x < p, on the curve, prime-order subgroup).  Throws Error naming the first invalid point.
+    static CommitKey from_slice(Context &ctx, const std::vector<uint8_t> &bytes) {
+        if (bytes.empty() || bytes.size() % 48) throw Error("CommitKey::from_slice: the length is not a positive multiple of 48");
+        const size_t n = bytes.size() / 48;
+        pb200_srs *srs = nullptr;
+        ctx.check(pb200_srs_from_compressed(ctx.raw(), bytes.data(), n, nullptr, &srs), "pb200_srs_from_compressed");
+        CommitKey ck(ctx, srs);
+        if (n <= ((size_t)1 << 22)) ctx.check(pb200_srs_precompute(ctx.raw(), srs), "pb200_srs_precompute");
+        return ck;
+    }
+    // CommitKey::to_var_bytes: the points as 48-byte compressed encodings, encoded on the device
+    std::vector<uint8_t> to_var_bytes() const {
+        const size_t n = pb200_srs_len(srs_);
+        std::vector<uint8_t> out(48 * n);
+        if (n) ctx_->check(pb200_srs_to_compressed(ctx_->raw(), srs_, 0, n, out.data()), "pb200_srs_to_compressed");
+        return out;
+    }
     CommitKey(CommitKey &&o) noexcept : ctx_(o.ctx_), srs_(o.srs_) { o.srs_ = nullptr; }
     CommitKey(const CommitKey &) = delete;
     ~CommitKey() {

@@ -20,6 +20,7 @@ EXPORTS = [
     "pb200_srs_upload", "pb200_srs_wrap_dev", "pb200_srs_precompute", "pb200_srs_free", "pb200_srs_len",
     "pb200_msm_g1", "pb200_msm_g1_dev", "pb200_msm_g1_batch_dev", "pb200_pippenger_g1", "pb200_g1_sum", "pb200_msm_window_bits",
     "pb200_srs_generate", "pb200_srs_generate_range", "pb200_srs_dev_ptr", "pb200_kzg_witness_dev", "pb200_fr_horner_step_dev",
+    "pb200_srs_from_compressed", "pb200_srs_to_compressed",
     "pb200_preprocess", "pb200_preprocess_sharded", "pb200_prover_key_free", "pb200_prover_key_size", "pb200_prover_key_bytes", "pb200_prove", "pb200_prove_dev",
     "pb200_transcript_selftest", "pb200_synthetic_circuit", "pb200_verify", "pb200_opening_key_from_tau",
     "pb200_pairing_selftest",
@@ -33,6 +34,10 @@ EXPORTS = [
 
 class Pb200Error(RuntimeError):
     pass
+
+
+# per-point status of pb200_srs_from_compressed (PB200_G1_* in include/pb200.h)
+G1_OK, G1_BAD_FLAGS, G1_X_RANGE, G1_NOT_ON_CURVE, G1_NOT_IN_SUBGROUP, G1_IDENTITY = range(6)
 
 
 ALLGATHER_FN = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t)
@@ -105,6 +110,8 @@ def lib():
         L.pb200_preprocess_sharded.argtypes = [vp, vp, ctypes.POINTER(Circuit), ctypes.c_char_p, ctypes.c_size_t, ctypes.POINTER(Shard),
                                                ctypes.POINTER(vp), vp]
         L.pb200_srs_generate_range.argtypes = [vp, u64p, ctypes.c_size_t, ctypes.c_size_t, ctypes.POINTER(vp)]
+        L.pb200_srs_from_compressed.argtypes = [vp, vp, ctypes.c_size_t, vp, ctypes.POINTER(vp)]
+        L.pb200_srs_to_compressed.argtypes = [vp, vp, ctypes.c_size_t, ctypes.c_size_t, vp]
         L.pb200_prover_key_free.argtypes = [vp, vp]
         L.pb200_prover_key_free.restype = None
         L.pb200_prover_key_size.argtypes = [vp]
@@ -325,6 +332,33 @@ class Context:
 
     def srs_dev_ptr(self, srs):
         return lib().pb200_srs_dev_ptr(srs)
+
+    def srs_from_compressed(self, data, status_out=None):
+        """`CommitKey::from_slice` on the device: 48-byte compressed points (bytes-like, length a positive multiple of 48) →
+        an SRS handle.  Every point is checked (flags, x < p, on the curve, prime-order subgroup); an invalid one raises
+        ValueError with the library's message, which names the first invalid index and the reason.  status_out (optional
+        uint8 array of one byte per point) receives G1_* per point, also when the call fails."""
+        buf = np.frombuffer(data, dtype=np.uint8)
+        if buf.size == 0 or buf.size % 48:
+            raise ValueError("compressed commit key: %d bytes is not a positive multiple of 48" % buf.size)
+        n = buf.size // 48
+        if status_out is not None:
+            assert status_out.dtype == np.uint8 and status_out.size == n and status_out.flags["C_CONTIGUOUS"]
+        h = ctypes.c_void_p()
+        rc = lib().pb200_srs_from_compressed(self._h, _ptr(buf), n, _ptr(status_out) if status_out is not None else None,
+                                             ctypes.byref(h))
+        if rc == 1:   # PB200_ERR_ARG: an invalid point (or argument) — a property of the input, not of the device
+            raise ValueError(lib().pb200_last_error(self._h).decode())
+        self._check(rc)
+        return h
+
+    def srs_to_compressed(self, srs, offset=0, n=None):
+        """`CommitKey::to_var_bytes` of points [offset, offset + n) (default: to the end): 48·n bytes."""
+        if n is None:
+            n = lib().pb200_srs_len(srs) - offset
+        out = np.empty(48 * n, np.uint8)
+        self._check(lib().pb200_srs_to_compressed(self._h, srs, offset, n, _ptr(out)))
+        return out.tobytes()
 
     def kzg_witness_dev(self, poly_dev, n, z_mont, quotient_dev):
         z = np.ascontiguousarray(z_mont, dtype=np.uint64).reshape(4)

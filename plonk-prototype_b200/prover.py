@@ -247,6 +247,25 @@ class PublicParameters:
         self.n_points = _native.lib().pb200_srs_len(self.srs)
         return self
 
+    def to_var_bytes(self):
+        """`PublicParameters::to_var_bytes`: opening key (240 bytes) ‖ commit key as 48-byte compressed points (encoded on
+        the GPU) — the distributable form, e.g. of a setup ceremony's output."""
+        from . import serial
+        return serial.opening_key_to_bytes(self.beta_h) + serial.commit_key_to_var_bytes(self.ctx, self.srs)
+
+    @classmethod
+    def from_slice(cls, data, ctx=None, precompute=True):
+        """`PublicParameters::from_slice`: parameters in the to_var_bytes form, checked.  β·H must be a point of G2 (host);
+        every commit-key point is decoded and checked on the GPU (flags, x < p, on the curve, prime-order subgroup).
+        ValueError on anything invalid; nothing stays allocated then."""
+        from . import serial
+        self = cls.__new__(cls)
+        self.ctx = ctx or default_context()
+        self.beta_h = serial.opening_key_from_bytes_checked(bytes(data[:serial.OPENING_KEY_SIZE]))
+        self.srs = serial.commit_key_from_slice(self.ctx, bytes(data[serial.OPENING_KEY_SIZE:]), precompute)
+        self.n_points = _native.lib().pb200_srs_len(self.srs)
+        return self
+
     def close(self):
         if self.srs is not None:
             self.ctx.srs_free(self.srs)

@@ -10,13 +10,16 @@ from memory of the crates —
   * `CommitKey::to_raw_bytes`: u64 LE point count ‖ the points' raw bytes;  `to_var_bytes`: the points compressed, no prefix;
   * `OpeningKey::to_bytes`: g (48, compressed G1) ‖ h (96, compressed G2) ‖ β·h (96) = 240 bytes;
   * `PublicParameters::to_raw_bytes` / `to_var_bytes`: the opening key, then the commit key.
-The point data never passes through Python integers in the raw form (numpy reshapes of the device image); the opening key's
-two G2 points do (compression needs canonical coordinates and a square root on the way back) — cold, three points per SRS."""
+The commit key's points never pass through Python integers: the raw form is a numpy reshape of the device image, the compressed
+form is encoded and decoded (with every check of `G1Affine::from_bytes`) on the GPU (`pb200_srs_{to,from}_compressed`).  The
+opening key's two G2 points do (compression needs canonical coordinates and a square root on the way back) — cold, three
+points per SRS."""
 import numpy as np
 
 from . import _native
 
 P = 0x1A0111EA397FE69A4B1BA7B6434BACD764774B84F38512BF6730D2A0F6B0F6241EABFFFEB153FFFFB9FEFFFFFFFFAAAB
+R = 0x73EDA753299D7D483339D80809A1D80553BDA402FFFE5BFEFFFFFFFF00000001
 _R_INV = pow(1 << 384, -1, P)
 G1_RAW_SIZE, G1_SIZE, G2_SIZE, OPENING_KEY_SIZE = 97, 48, 96, 240
 # the generators' compressed encodings (zcash format; SURVEY.md App. A.3-A.4)
@@ -93,6 +96,61 @@ def g2_from_bytes(b):
     return np.array(_int_to_limbs_mont(x[0]) + _int_to_limbs_mont(x[1]) + _int_to_limbs_mont(y[0]) + _int_to_limbs_mont(y[1]), dtype=np.uint64)
 
 
+def _fp2_inv(a):
+    t = pow((a[0] * a[0] + a[1] * a[1]) % P, -1, P)
+    return (a[0] * t % P, (-a[1]) * t % P)
+
+
+def _g2_add(p, q):
+    """Affine addition on the twist over Fp2; None is the identity."""
+    if p is None:
+        return q
+    if q is None:
+        return p
+    if p[0] == q[0]:
+        if ((p[1][0] + q[1][0]) % P, (p[1][1] + q[1][1]) % P) == (0, 0):
+            return None
+        xx = _fp2_mul(p[0], p[0])
+        lam = _fp2_mul((3 * xx[0] % P, 3 * xx[1] % P), _fp2_inv((2 * p[1][0] % P, 2 * p[1][1] % P)))
+    else:
+        lam = _fp2_mul(((q[1][0] - p[1][0]) % P, (q[1][1] - p[1][1]) % P), _fp2_inv(((q[0][0] - p[0][0]) % P, (q[0][1] - p[0][1]) % P)))
+    ll = _fp2_mul(lam, lam)
+    x3 = ((ll[0] - p[0][0] - q[0][0]) % P, (ll[1] - p[0][1] - q[0][1]) % P)
+    t = _fp2_mul(lam, ((p[0][0] - x3[0]) % P, (p[0][1] - x3[1]) % P))
+    return (x3, ((t[0] - p[1][0]) % P, (t[1] - p[1][1]) % P))
+
+
+def g2_from_bytes_checked(b):
+    """`G2Affine::from_bytes` with every check: flags, x.c0 and x.c1 < p, on the twist, and r·Q = O (the order-r subgroup;
+    double-and-add over Fp2 on Python integers — cold, one point).  The identity is rejected: an opening key's β·H never is.
+    → 24 u64 (x.c0 ‖ x.c1 ‖ y.c0 ‖ y.c1, Montgomery); ValueError on anything invalid."""
+    if len(b) != G2_SIZE or not b[0] & 0x80:
+        raise ValueError("G2 point: not a 96-byte compressed encoding")
+    if b[0] & 0x40:
+        raise ValueError("G2 point: the identity")
+    x1 = int.from_bytes(bytes([b[0] & 0x1F]) + b[1:48], "big")
+    x0 = int.from_bytes(b[48:], "big")
+    if x0 >= P or x1 >= P:
+        raise ValueError("G2 point: x is not below p")
+    x = (x0, x1)
+    rhs = _fp2_mul(_fp2_mul(x, x), x)
+    y = _fp2_sqrt(((rhs[0] + 4) % P, (rhs[1] + 4) % P))
+    if y is None:
+        raise ValueError("G2 point: not on the curve")
+    larger = y[1] > (P - 1) // 2 if y[1] else y[0] > (P - 1) // 2
+    if larger != bool(b[0] & 0x20):
+        y = ((-y[0]) % P, (-y[1]) % P)
+    acc, add, k = None, (x, y), R
+    while k:
+        if k & 1:
+            acc = _g2_add(acc, add)
+        add = _g2_add(add, add)
+        k >>= 1
+    if acc is not None:
+        raise ValueError("G2 point: not in the prime-order subgroup")
+    return np.array(_int_to_limbs_mont(x[0]) + _int_to_limbs_mont(x[1]) + _int_to_limbs_mont(y[0]) + _int_to_limbs_mont(y[1]), dtype=np.uint64)
+
+
 def opening_key_to_bytes(beta_h):
     """`OpeningKey::to_bytes` for the opening key (G, H, β·H) of a trapdoor-generated SRS (`_native.opening_key_from_tau`)."""
     return G1_GENERATOR_BYTES + G2_GENERATOR_BYTES + g2_to_bytes(beta_h)
@@ -104,6 +162,16 @@ def opening_key_from_bytes(b):
     if b[:48] != G1_GENERATOR_BYTES or b[48:144] != G2_GENERATOR_BYTES:
         raise ValueError("opening key over other generators than the BLS12-381 ones")
     return g2_from_bytes(b[144:])
+
+
+def opening_key_from_bytes_checked(b):
+    """The opening key of `PublicParameters::from_slice`: as opening_key_from_bytes, and β·H must be a valid point of G2
+    (g2_from_bytes_checked).  ValueError on anything invalid."""
+    if len(b) != OPENING_KEY_SIZE:
+        raise ValueError("opening key: %d bytes, expected %d" % (len(b), OPENING_KEY_SIZE))
+    if b[:48] != G1_GENERATOR_BYTES or b[48:144] != G2_GENERATOR_BYTES:
+        raise ValueError("opening key over other generators than the BLS12-381 ones")
+    return g2_from_bytes_checked(bytes(b[144:]))
 
 
 # ---- commit key ---------------------------------------------------------------------------------------------------------
@@ -134,11 +202,24 @@ def commit_key_from_slice_unchecked(ctx, b, precompute=True):
 
 
 def commit_key_to_var_bytes(ctx, srs):
-    """`CommitKey::to_var_bytes`: compressed points (canonical coordinates need one host pass per point — meant for small keys)."""
-    from .msm import g1_to_bytes
+    """`CommitKey::to_var_bytes`: the points compressed (48 bytes each, no prefix), encoded on the GPU."""
     n = _native.lib().pb200_srs_len(srs)
-    pts = np.empty((n, 12), np.uint64)
-    if n:
-        ctx.d2h(pts, ctx.srs_dev_ptr(srs))
-    one = np.array([0x760900000002FFFD, 0xEBF4000BC40C0002, 0x5F48985753C758BA, 0x77CE585370525745, 0x5C071A97A256EC6D, 0x15F65EC3FA80E493], np.uint64)
-    return b"".join(g1_to_bytes(np.concatenate([p, one])) for p in pts)   # (x, y, 1) in Montgomery form
+    return ctx.srs_to_compressed(srs) if n else b""
+
+
+def commit_key_from_slice(ctx, b, precompute=True):
+    """`CommitKey::from_slice` → an SRS handle resident on the GPU.  Every point is decoded and checked on the device as
+    `G1Affine::from_bytes` does (flags, x < p, on the curve, prime-order subgroup); ValueError names the first invalid one.
+    Keys of up to 2^22 points also get their pre-doubled window copies, as commit_key_from_slice_unchecked."""
+    b = bytes(b)
+    if not b or len(b) % G1_SIZE:
+        raise ValueError("CommitKey: %d bytes is not a positive multiple of %d" % (len(b), G1_SIZE))
+    srs = ctx.srs_from_compressed(b)
+    n = len(b) // G1_SIZE
+    if precompute and n <= (1 << 22):
+        try:
+            ctx.srs_precompute(srs)
+        except Exception:
+            ctx.srs_free(srs)
+            raise
+    return srs
