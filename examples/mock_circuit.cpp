@@ -81,6 +81,12 @@ int main() {
         ProofBytes tampered = proof;
         tampered[600] ^= 1;
         CHECK(!verify_proof(prover.verifier_key(), prover.padded_size(), label, tampered, cs.public_inputs_sparse_store(), tau));
+        {  // the valid and the two invalid cases above, verified in one batch on the GPU
+            const std::array<uint8_t, 32> seed{0x5e, 0xed};
+            const std::vector<bool> verdicts = verify_proofs(ctx, prover.verifier_key(), prover.padded_size(), label, {proof, proof, tampered},
+                                                             {cs.public_inputs_sparse_store(), wrong, cs.public_inputs_sparse_store()}, tau, seed);
+            CHECK(verdicts == std::vector<bool>({true, false, false}));
+        }
 
         // MockCircuit::prove_ownership (/root/reference/src/zk/circuits.rs:63-66): sk·G computed in circuit by the fixed-base
         // widget equals the public key, which enters as two public inputs

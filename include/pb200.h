@@ -285,6 +285,32 @@ PB200_API int pb200_prove_dev(pb200_ctx *ctx, const pb200_srs *srs, pb200_prover
 PB200_API int pb200_verify(const uint8_t vk_commitments[15 * 48], size_t n, const uint8_t *transcript_label, size_t label_len,
                            const uint8_t proof[1040], const uint32_t *pi_gate, const uint64_t *pi_mont, size_t n_pi,
                            const uint64_t beta_h[24], int *accepted);
+/* Many proofs of ONE circuit in one batched check on the GPU (dusk-plonk 0.8 has no multi-proof API; this is the
+ * standard random-linear-combination batch of Proof::verify).  One verifier key, label and padded size n as for
+ * pb200_verify; proofs: n_proofs × 1040 bytes back to back; pi_gate (n_pi entries) is shared by every proof and
+ * pi_mont holds n_proofs × n_pi × 4 u64 Montgomery values, proof-major.
+ *   accepted[k] (out, n_proofs bytes) = what pb200_verify returns for proof k with its public inputs: a valid proof is
+ *   never rejected; an invalid one is accepted with probability about 1/r per pairing check.  *all_accepted = 1 iff
+ *   every accepted[k] is 1.  Verdicts are deterministic for a given seed (32 bytes; callers draw it at random).
+ * Errors: PB200_ERR_ARG for a null pointer (seed included), n not a power of two in [2, 2^30], a duplicate pi_gate,
+ *   pi_gate[j] ≥ n, β·H not on the curve, n_proofs = 0 or n_proofs > 2^20 — all checked before any proof is looked at.
+ *   A malformed verifier key rejects every proof (not an error).  A proof with a point that fails G1Affine::from_bytes, an
+ *   evaluation ≥ r, z_H(z) = 0, z = 1 or z = ω^g for a public-input gate g is rejected and left out of the combination.
+ *   The identity encoding c0 00…00 is a valid proof point and contributes zero.  Nothing stays allocated on return.
+ * Algorithm: each proof's equation e(−W_k, βH)·e(C_k, H) = 1 has C_k, W_k linear in its 11 points and in 16 shared
+ *   bases (the 15 key commitments and G), with scalars from its own transcript (derived on the device, one thread per
+ *   proof).  Weights: per proof, after the transcript's challenge u, its public inputs are appended ("pi", one scalar
+ *   each) and 32 bytes drawn ("batch digest") = d_k; on the host D = Merlin("pb200 verify_batch") absorbing seed, n,
+ *   n_proofs and d_0‖…‖d_{K−1} ("seed", "n", "K", "digests"; challenge "D"); ρ_k = Merlin("pb200 rho") absorbing D ("D")
+ *   and k ("k"), challenge scalar "rho".  Then e(−Σρ_kW_k, βH)·e(Σρ_kC_k, H) = 1 is one pairing check on the host over
+ *   two MSMs on the device.  If it fails, bisection over contiguous proof ranges (same ρ_k) finds the invalid proofs:
+ *   an all-valid batch costs exactly one pairing check, b invalid proofs at most about 1 + 2·b·⌈log2 K⌉.
+ * With profiling on, pb200_profile_sum_ms knows "verify.decompress", "verify.prepare", "verify.weight" (kernel time),
+ *   "verify.msm" (device time of the call's MSMs) and "verify.pairing" (host wall clock, one sample per pairing check).
+ * Blocks. */
+PB200_API int pb200_verify_batch(pb200_ctx *ctx, const uint8_t vk_commitments[15 * 48], size_t n, const uint8_t *transcript_label,
+                                 size_t label_len, const uint8_t *proofs, size_t n_proofs, const uint32_t *pi_gate, const uint64_t *pi_mont,
+                                 size_t n_pi, const uint64_t beta_h[24], const uint8_t seed[32], uint8_t *accepted, int *all_accepted);
 /* β·H for parameters generated from a known trapdoor (pb200_srs_generate): the G2 half of PublicParameters::setup. */
 PB200_API int pb200_opening_key_from_tau(const uint64_t tau_mont[4], uint64_t beta_h_out[24]);
 /* Pairing self-check without a known-answer table: e(a·G1, b·G2) = e(G1, G2)^(ab) ≠ 1. */

@@ -553,4 +553,34 @@ inline bool verify_proof(const VerifierKeyBytes &vk, size_t padded_size, const s
     return accepted != 0;
 }
 
+// Many proofs of one circuit in one batched check on the GPU (pb200_verify_batch): verdict k is what verify_proof returns
+// for proofs[k] with public_inputs[k].  Every proof's public inputs must sit at the same gates.  seed: 32 random bytes.
+inline std::vector<bool> verify_proofs(Context &ctx, const VerifierKeyBytes &vk, size_t padded_size, const std::string &label,
+                                       const std::vector<ProofBytes> &proofs, const std::vector<std::map<uint32_t, BlsScalar>> &public_inputs,
+                                       const BlsScalar &tau, const std::array<uint8_t, 32> &seed) {
+    if (proofs.size() != public_inputs.size() || proofs.empty()) throw Error("verify_proofs: one public-input map per proof");
+    uint64_t beta_h[24];
+    if (pb200_opening_key_from_tau(tau.v.l, beta_h) != 0) throw Error("pb200_opening_key_from_tau");
+    std::vector<uint32_t> pos;
+    for (const auto &kv : public_inputs[0]) pos.push_back(kv.first);
+    std::vector<BlsScalar> val;
+    std::vector<uint8_t> bytes;
+    for (size_t k = 0; k < proofs.size(); k++) {
+        if (public_inputs[k].size() != pos.size()) throw Error("verify_proofs: public inputs at different gates");
+        size_t j = 0;
+        for (const auto &kv : public_inputs[k]) {
+            if (kv.first != pos[j++]) throw Error("verify_proofs: public inputs at different gates");
+            val.push_back(kv.second);
+        }
+        bytes.insert(bytes.end(), proofs[k].begin(), proofs[k].end());
+    }
+    std::vector<uint8_t> accepted(proofs.size());
+    int all = 0;
+    ctx.check(pb200_verify_batch(ctx.raw(), vk.data(), padded_size, reinterpret_cast<const uint8_t *>(label.data()), label.size(),
+                                 bytes.data(), proofs.size(), pos.data(), reinterpret_cast<const uint64_t *>(val.data()), pos.size(), beta_h,
+                                 seed.data(), accepted.data(), &all),
+              "pb200_verify_batch");
+    return std::vector<bool>(accepted.begin(), accepted.end());
+}
+
 }  // namespace pb200

@@ -1,6 +1,6 @@
 """plonk-prototype_b200 — B200-native MSM / NTT backend behind the dusk-plonk / dusk-bls12_381 API
 surface that Manta-Network/Plonk-Prototype's circuits prove through.  See DESIGN.md."""
-from ._native import Context, Pb200Error, LIB_PATH, EXPORTS, verify, opening_key_from_tau  # noqa: F401
+from ._native import Context, Pb200Error, LIB_PATH, EXPORTS, verify, verify_batch, opening_key_from_tau  # noqa: F401
 from .domain import EvaluationDomain, Polynomial, Evaluations, InvalidEvalDomainSize, default_context  # noqa: F401
 from .msm import msm_variable_base, pippenger, CommitKey, g1_to_bytes  # noqa: F401
 from .dist_ntt import DistributedDomain, ShardSpec, GpuBackend, PeerBuffers  # noqa: F401

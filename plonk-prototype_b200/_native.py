@@ -22,7 +22,7 @@ EXPORTS = [
     "pb200_srs_generate", "pb200_srs_generate_range", "pb200_srs_dev_ptr", "pb200_kzg_witness_dev", "pb200_fr_horner_step_dev",
     "pb200_srs_from_compressed", "pb200_srs_to_compressed",
     "pb200_preprocess", "pb200_preprocess_sharded", "pb200_prover_key_free", "pb200_prover_key_size", "pb200_prover_key_bytes", "pb200_prove", "pb200_prove_dev",
-    "pb200_transcript_selftest", "pb200_synthetic_circuit", "pb200_verify", "pb200_opening_key_from_tau",
+    "pb200_transcript_selftest", "pb200_synthetic_circuit", "pb200_verify", "pb200_verify_batch", "pb200_opening_key_from_tau",
     "pb200_pairing_selftest",
     "pb200_synthetic_bases_dev", "pb200_profile_enable", "pb200_profile_ms", "pb200_profile_reset", "pb200_profile_sum_ms",
     "pb200_launch_count",
@@ -124,6 +124,8 @@ def lib():
                                                 ctypes.c_char_p, ctypes.c_size_t]
         L.pb200_verify.argtypes = [vp, ctypes.c_size_t, ctypes.c_char_p, ctypes.c_size_t, vp, vp, u64p, ctypes.c_size_t, u64p,
                                    ctypes.POINTER(ctypes.c_int)]
+        L.pb200_verify_batch.argtypes = [vp, vp, ctypes.c_size_t, ctypes.c_char_p, ctypes.c_size_t, vp, ctypes.c_size_t, vp, u64p,
+                                         ctypes.c_size_t, u64p, vp, vp, ctypes.POINTER(ctypes.c_int)]
         L.pb200_opening_key_from_tau.argtypes = [u64p, u64p]
         L.pb200_pairing_selftest.argtypes = [u64p, u64p, ctypes.POINTER(ctypes.c_int)]
         L.pb200_synthetic_circuit.argtypes = [ctypes.c_size_t, ctypes.c_uint64, ctypes.c_uint32, ctypes.POINTER(vp), ctypes.POINTER(vp), u64p,
@@ -180,6 +182,31 @@ def verify(vk_bytes, n, label, proof, pi_gate, pi_mont, beta_h):
     if rc != 0:
         raise Pb200Error("pb200_verify: bad argument (%d)" % rc)
     return bool(ok.value)
+
+
+def verify_batch(ctx, vk_bytes, n, label, proofs, pi_gate, pi_mont, beta_h, seed=None):
+    """Many proofs of one circuit in one batched check on the GPU (pb200_verify_batch).  proofs: a sequence of 1040-byte
+    proofs (or their concatenation); pi_gate: the n_pi gates every proof's public inputs sit at; pi_mont: (K, n_pi, 4)
+    uint64 Montgomery values; seed: 32 bytes, drawn from os.urandom when None.  Returns a numpy bool array, entry k being
+    what `verify` returns for proof k."""
+    h = ctx._h if isinstance(ctx, Context) else ctx
+    vk = np.frombuffer(bytes(vk_bytes), dtype=np.uint8).copy()
+    pr = np.frombuffer(b"".join(bytes(p) for p in proofs) if not isinstance(proofs, (bytes, bytearray)) else bytes(proofs),
+                       dtype=np.uint8).copy()
+    assert vk.size == 720 and pr.size % 1040 == 0
+    K = pr.size // 1040
+    pos = np.ascontiguousarray(pi_gate, dtype=np.uint32).reshape(-1)
+    piv = np.ascontiguousarray(pi_mont, dtype=np.uint64).reshape(K, pos.size, 4) if pos.size else np.zeros((K, 0, 4), np.uint64)
+    bh = np.ascontiguousarray(beta_h, dtype=np.uint64).reshape(24)
+    sd = np.frombuffer(os.urandom(32) if seed is None else bytes(seed), dtype=np.uint8).copy()
+    assert sd.size == 32
+    acc = np.zeros(max(K, 1), np.uint8)
+    all_ok = ctypes.c_int(0)
+    rc = lib().pb200_verify_batch(h, _ptr(vk), n, bytes(label), len(label), _ptr(pr) if K else None, K, _ptr(pos) if pos.size else None,
+                                  _ptr(piv) if pos.size else None, pos.size, _ptr(bh), _ptr(sd), _ptr(acc), ctypes.byref(all_ok))
+    if rc != 0:
+        raise Pb200Error("pb200_verify_batch failed (%d): %s" % (rc, lib().pb200_last_error(h).decode()))
+    return acc[:K].astype(bool)
 
 
 class Context:
@@ -524,6 +551,11 @@ class Context:
 
     def synthetic_bases_dev(self, dev, n, a=0xB2000001, d=0x9E3779B1):
         self._check(lib().pb200_synthetic_bases_dev(self._h, ctypes.c_void_p(dev), n, a, d))
+
+    # -- batched verification
+    def verify_batch(self, vk_bytes, n, label, proofs, pi_gate, pi_mont, beta_h, seed=None):
+        """`verify_batch` on this context."""
+        return verify_batch(self, vk_bytes, n, label, proofs, pi_gate, pi_mont, beta_h, seed)
 
     # -- measurement
     def profile_enable(self, on=True):

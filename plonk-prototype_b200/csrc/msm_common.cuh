@@ -79,6 +79,10 @@ int tail_g1_normalize(pb200_ctx *ctx, const uint32_t *xyz, const uint64_t *scala
 int tail_precompute(pb200_ctx *ctx, const G1Affine *bases, uint32_t n, uint32_t c, uint32_t W, G1Affine *pre);
 int tail_synthetic_bases(pb200_ctx *ctx, G1Affine *out, uint64_t n, uint64_t a, uint64_t d);
 
+// ---- checked compressed-point decoder (srs_io.cu): G1Affine::from_bytes, one thread per point, 128 threads per block
+__global__ void g1_decompress_kernel(const uint4 *__restrict__ enc, uint32_t n, G1Affine *__restrict__ out, uint8_t *__restrict__ status,
+                                     uint32_t *first_bad);
+
 // ------------------------------------------------------------------------------------ accumulate
 // Output rule shared by every level.  A run that lies strictly inside its segment is complete and
 // goes to its bucket.  A run that touches the left (right) segment boundary *and* continues in the

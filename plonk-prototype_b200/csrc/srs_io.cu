@@ -9,10 +9,9 @@
 #include "g1_codec.cuh"
 #include "msm_common.cuh"
 
-namespace {
-
 // One thread per point: three 16-byte loads, decode + checks, one 96-byte store of the packed affine point.  An invalid
 // point is an ordinary result: its status is written and its index folded into *first_bad; the thread returns normally.
+// Also launched by the batched verifier (verify_batch.cu) on the points of its proofs and verifier key.
 __global__ void __launch_bounds__(128) g1_decompress_kernel(const uint4 *__restrict__ enc, uint32_t n, G1Affine *__restrict__ out,
                                                             uint8_t *__restrict__ status, uint32_t *first_bad) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -28,6 +27,9 @@ __global__ void __launch_bounds__(128) g1_decompress_kernel(const uint4 *__restr
         atomicMin(first_bad, i);
     }
 }
+
+namespace {
+
 // One thread per point: one 96-byte load, two conversions out of Montgomery form, three 16-byte stores.
 __global__ void __launch_bounds__(256) g1_compress_kernel(const G1Affine *__restrict__ pts, uint32_t n, uint4 *__restrict__ enc) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
