@@ -111,6 +111,12 @@ PB200_API int pb200_srs_wrap_dev(pb200_ctx *ctx, const uint64_t *xy_mont_dev, si
  * all Pippenger windows share one bucket set — no per-window reduction and no Horner pass, which is what bounds
  * prover-size (2^16…2^22) MSMs.  Costs W ≈ 12-13 times the SRS memory; results are unchanged. */
 PB200_API int pb200_srs_precompute(pb200_ctx *ctx, pb200_srs *srs);
+/* The commit key in the Lagrange basis of the domain of n = 2^log_n points: *out holds Q_i = [L_i(τ)]G = n⁻¹·Σ_j ω^(−ij)·P_j,
+ * i < n, computed on the device from the first n points of `srs` (an inverse NTT over G1: no trapdoor needed), so that
+ * Σ_i f(ω^i)·Q_i is the commitment to the polynomial f of degree < n from its evaluations.  log_n ≤ 26, n ≤ pb200_srs_len.
+ * A key that is not powers of τ can give an identity point: PB200_ERR_ARG, nothing allocated.  Free with pb200_srs_free.
+ * pb200_preprocess builds one for its domain itself (see there). */
+PB200_API int pb200_srs_lagrange(pb200_ctx *ctx, const pb200_srs *srs, uint32_t log_n, pb200_srs **out);
 PB200_API void pb200_srs_free(pb200_ctx *ctx, pb200_srs *srs);
 PB200_API size_t pb200_srs_len(const pb200_srs *srs);
 /* msm_variable_base(&points[offset .. offset + n], scalars): Σ scalars[i]·points[offset + i].
@@ -199,7 +205,11 @@ typedef struct pb200_circuit {
  * the verifier key.  Everything stays resident in HBM behind the returned handle.  vk_commitments (optional) receives
  * the 15 compressed commitments in the column order above followed by left/right/out/fourth sigma.
  * Widgets: arithmetic, range, logic, fixed-base scalar multiplication and variable-base point addition on JubJub (all
- * eleven selector columns of StandardComposer). */
+ * eleven selector columns of StandardComposer).
+ * On one GPU, with n ≤ 2^22 and a commit key that has pre-doubled copies (pb200_srs_precompute), the key also holds the
+ * Lagrange-basis key of its domain (pb200_srs_lagrange) with its own pre-doubled copies — (W + 1)·n·96 bytes, 1.3 GiB at
+ * n = 2^20 — and pb200_prove commits the wire polynomials from their evaluations, whose zero and small values cost almost
+ * nothing in the MSM.  The proof bytes are the same.  Environment PB200_LAGRANGE_COMMIT=0, read here, leaves it out. */
 PB200_API int pb200_preprocess(pb200_ctx *ctx, const pb200_srs *srs, const pb200_circuit *circuit, const uint8_t *transcript_label,
                                size_t label_len, pb200_prover_key **out, uint8_t vk_commitments[15 * 48]);
 PB200_API void pb200_prover_key_free(pb200_ctx *ctx, pb200_prover_key *pk);

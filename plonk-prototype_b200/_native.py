@@ -17,7 +17,7 @@ EXPORTS = [
     "pb200_malloc", "pb200_free", "pb200_h2d", "pb200_d2h",
     "pb200_domain_log_size", "pb200_ntt", "pb200_ntt_dev", "pb200_ntt_batch_dev", "pb200_ntt_columns_dev", "pb200_ntt_columns_scatter_dev",
     "pb200_ipc_export", "pb200_ipc_open", "pb200_ipc_close", "pb200_block_transpose_dev",
-    "pb200_srs_upload", "pb200_srs_wrap_dev", "pb200_srs_precompute", "pb200_srs_free", "pb200_srs_len",
+    "pb200_srs_upload", "pb200_srs_wrap_dev", "pb200_srs_precompute", "pb200_srs_lagrange", "pb200_srs_free", "pb200_srs_len",
     "pb200_msm_g1", "pb200_msm_g1_dev", "pb200_msm_g1_batch_dev", "pb200_pippenger_g1", "pb200_g1_sum", "pb200_msm_window_bits",
     "pb200_srs_generate", "pb200_srs_generate_range", "pb200_srs_dev_ptr", "pb200_kzg_witness_dev", "pb200_fr_horner_step_dev",
     "pb200_srs_from_compressed", "pb200_srs_to_compressed",
@@ -90,6 +90,7 @@ def lib():
         L.pb200_srs_upload.argtypes = [vp, u64p, ctypes.c_size_t, ctypes.POINTER(vp)]
         L.pb200_srs_wrap_dev.argtypes = [vp, u64p, ctypes.c_size_t, ctypes.POINTER(vp)]
         L.pb200_srs_precompute.argtypes = [vp, vp]
+        L.pb200_srs_lagrange.argtypes = [vp, vp, ctypes.c_uint32, ctypes.POINTER(vp)]
         L.pb200_srs_free.argtypes = [vp, vp]
         L.pb200_srs_free.restype = None
         L.pb200_srs_len.argtypes = [vp]
@@ -309,6 +310,12 @@ class Context:
 
     def srs_precompute(self, srs):
         self._check(lib().pb200_srs_precompute(self._h, srs))
+
+    def srs_lagrange(self, srs, log_n):
+        """New commit key [L_i(τ)]G, i < 2^log_n, in the Lagrange basis of the domain of size 2^log_n (pb200_srs_lagrange)."""
+        h = ctypes.c_void_p()
+        self._check(lib().pb200_srs_lagrange(self._h, srs, log_n, ctypes.byref(h)))
+        return h
 
     def srs_free(self, srs):
         lib().pb200_srs_free(self._h, srs)

@@ -128,3 +128,6 @@ int kzg_witness_slice_phase1(pb200_ctx *ctx, const uint64_t *poly_slice_dev, uin
 int kzg_witness_slice_phase2(pb200_ctx *ctx, uint32_t lo, uint32_t cnt, uint64_t *q_slice_dev, uint64_t *work_dev,
                              const uint64_t later_slices_total[4]);
 size_t kzg_witness_slice_work_scalars(uint32_t cnt);
+// lagrange.cu: Lagrange-basis key [L_i(τ)]G, i < 2^log_n, from the first 2^log_n points of `srs` (owned, no pre-doubled
+// copies).  *degenerate (and *out = nullptr, return 0) when some point is the identity, i.e. `srs` is not powers of τ.
+int lagrange_srs_build(pb200_ctx *ctx, const pb200_srs *srs, uint32_t log_n, pb200_srs **out, bool *degenerate);

@@ -163,6 +163,13 @@ struct El {
 typedef El<4> HFr;
 typedef El<6> HFp;
 
+// ω_n for n = 2^log_n (log_n ≤ 32): the generator of EvaluationDomain::new(n), the root every transform of the prover uses.
+inline HFr domain_root(uint32_t log_n) {
+    const uint64_t root32[4] = {0xb9b58d8c5f0e466aull, 0x5b1b4c801819d7ecull, 0x0af53ae352a31e64ull, 0x5bf3adda19e9b27bull};  // ω₃₂·R
+    HFr w = HFr::load(root32);
+    for (uint32_t k = log_n; k < 32; k++) w = w.sqr();
+    return w;
+}
 // BlsScalar::to_bytes: canonical value, 32 bytes little-endian.
 inline void fr_to_bytes(const HFr &a, uint8_t out[32]) {
     HFr c = a.from_mont();

@@ -408,6 +408,10 @@ struct pb200_prover_key {
     Fr *sig_evals = nullptr, *sig_poly = nullptr, *sig_4n = nullptr;  // 4·n, 4·n, 4·4n
     Fr *roots = nullptr, *lin_4n = nullptr, *l1_4n = nullptr;  // ω^i | X on the coset | L₁ on the coset
     uint32_t *wires = nullptr;
+    // Lagrange-basis commit key of this domain with its pre-doubled copies (lagrange.cu): round 1 commits the wire
+    // evaluations against it.  nullptr: the wires are committed from their coefficients against the caller's key.
+    pb200_srs *lagrange = nullptr;
+    size_t lagrange_bytes = 0;
     // prove workspace
     Fr *values = nullptr, *w_evals = nullptr, *w_poly = nullptr, *z_poly = nullptr, *pi_poly = nullptr, *ev4 = nullptr, *t_poly = nullptr,
        *lin_poly = nullptr, *agg = nullptr, *wit = nullptr, *num = nullptr, *den = nullptr, *small = nullptr;
@@ -584,11 +588,12 @@ extern "C" void pb200_prover_key_free(pb200_ctx *ctx, pb200_prover_key *pk) {
         if (pk->peer_slab[h] && h != pk->shard.rank) cudaIpcCloseMemHandle(pk->peer_slab[h]);
     cudaFree(pk->slab);
     cudaFree(pk->pi_pos);
+    pb200_srs_free(ctx, pk->lagrange);
     delete pk->seeded;
     delete pk;
 }
 extern "C" size_t pb200_prover_key_size(const pb200_prover_key *pk) { return pk ? pk->n : 0; }
-extern "C" size_t pb200_prover_key_bytes(const pb200_prover_key *pk) { return pk ? pk->slab_bytes : 0; }
+extern "C" size_t pb200_prover_key_bytes(const pb200_prover_key *pk) { return pk ? pk->slab_bytes + pk->lagrange_bytes : 0; }
 
 extern "C" int pb200_preprocess(pb200_ctx *ctx, const pb200_srs *srs, const pb200_circuit *circuit, const uint8_t *transcript_label,
                                 size_t label_len, pb200_prover_key **out, uint8_t vk_commitments[15 * 48]) {
@@ -682,12 +687,8 @@ extern "C" int pb200_preprocess_sharded(pb200_ctx *ctx, const pb200_srs *srs, co
 
     // domain constants on the host
     {
-        uint64_t root32[4] = {0xb9b58d8c5f0e466aull, 0x5b1b4c801819d7ecull, 0x0af53ae352a31e64ull, 0x5bf3adda19e9b27bull};  // ω₃₂·R
-        HFr w = HFr::load(root32);
-        HFr w4 = w;
-        for (uint32_t k = 0; k < 32 - log_n; k++) w = w.sqr();
-        for (uint32_t k = 0; k < 32 - (log_n + 2); k++) w4 = w4.sqr();
-        pk->omega = w;
+        const HFr w4 = hostf::domain_root(log_n + 2);
+        pk->omega = hostf::domain_root(log_n);
         pk->omega4 = w4;
         // 1 / ((7·ω_4n^i)^n − 1), i mod 4:  7^n · (ω_4n^n)^i − 1
         const HFr g = HFr::from_u64(7), gn = g.pow_u64(n), i4 = w4.pow_u64(n), one = HFr::one();
@@ -749,6 +750,18 @@ extern "C" int pb200_preprocess_sharded(pb200_ctx *ctx, const pb200_srs *srs, co
     PK_LAUNCHED();
     PK_TRY(coset_extend(ctx, pk->l1_4n, pk->lin_poly, (uint32_t)n, log_n + 2, 1));
     PK_CUDA(cudaStreamSynchronize(st));
+
+    // Lagrange-basis key for round 1: one GPU, a commit key with pre-doubled copies (the batched MSM needs them) and a
+    // domain whose copies fit (n ≤ 2^22, like pb200_srs_precompute).  PB200_LAGRANGE_COMMIT=0 keeps the monomial path.
+    const char *lag_env = getenv("PB200_LAGRANGE_COMMIT");
+    if (world == 1 && log_n <= 22 && srs->pre != nullptr && !(lag_env && strcmp(lag_env, "0") == 0)) {
+        bool degenerate = false;  // some L_i(τ) = 0: not a powers-of-τ key; the monomial path still commits correctly
+        PK_TRY(lagrange_srs_build(ctx, srs, log_n, &pk->lagrange, &degenerate));
+        if (pk->lagrange) {
+            PK_TRY(pb200_srs_precompute(ctx, pk->lagrange));
+            pk->lagrange_bytes = n * 96 * (1 + pk->lagrange->W_pre);  // affine points + their pre-doubled copies
+        }
+    }
 
     // Transcript::new(label) seeded with the verifier key
     pk->seeded = new merlin::Transcript(transcript_label, label_len);
@@ -812,7 +825,10 @@ static int prove_impl(pb200_ctx *ctx, const pb200_srs *srs, pb200_prover_key *pk
     PB_CUDA(ctx, cudaMemcpyAsync(pk->w_poly, pk->w_evals, 4 * n * sizeof(Fr), cudaMemcpyDeviceToDevice, st));
     PB_TRY(pb200_ntt_batch_dev(ctx, (uint64_t *)pk->w_poly, log_n, 4, 1, 0));
     const char *const w_label[4] = {"w_l", "w_r", "w_o", "w_4"};
-    PB_TRY(commit_bytes_batch(ctx, srs, pk, pk->w_poly, n, 4, n, P));
+    // Σ_i w(ω^i)·[L_i(τ)]G = [w(τ)]G: the evaluations are mostly zero or small (d is zero off a few rows, padding rows
+    // are zero), and a zero or small scalar costs no or one MSM entry where its coefficient form costs 13
+    if (pk->lagrange) PB_TRY(commit_bytes_batch(ctx, pk->lagrange, pk, pk->w_evals, n, 4, n, P));
+    else PB_TRY(commit_bytes_batch(ctx, srs, pk, pk->w_poly, n, 4, n, P));
     for (int c = 0; c < 4; c++) tr.append_commitment(w_label[c], P + 48 * c);
     clk.lap("prove.round1");
 
