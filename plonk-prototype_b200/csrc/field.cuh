@@ -20,6 +20,8 @@ template <class P>
 __device__ __noinline__ Field<P> field_mul_noinline(Field<P> a, Field<P> b);  // operands travel in registers
 template <class P>
 __device__ __noinline__ Field<P> field_sqr_noinline(Field<P> a);
+template <class P>
+__device__ __noinline__ Field<P> field_mul2_sum_noinline(Field<P> a, Field<P> b, Field<P> c, Field<P> d);
 #endif
 
 template <class P>
@@ -169,10 +171,10 @@ struct Field {
         }
         O[H - 1] = cc::pack64(cc::lo32(O[H - 1]), cc::addc(cc::hi32(O[H - 1]), 0));
     }
-    // Round i ≥ 1.  On entry position 0 of S is zero and the value (already divided by 2^32) is
+    // Start of round i ≥ 1.  On entry position 0 of S is zero and the value (already divided by 2^32) is
     // (S >> 32) + D·(one position down).  S's position 1 is folded into D's position 0, S is rebuilt
-    // one column lower as the new odd accumulator, D becomes the new even accumulator.
-    PB_HD static void round(uint64_t *S, uint64_t *D, const uint32_t *a, uint32_t bi) {
+    // one column lower as the new odd accumulator, D becomes the new even accumulator; a·b_i is added.
+    PB_HD static void shift_add_row(uint64_t *S, uint64_t *D, const uint32_t *a, uint32_t bi) {
         uint32_t d0 = cc::add_cc(cc::lo32(D[0]), cc::hi32(S[0]));  // carry → start of the odd chain
 #pragma unroll
         for (int k = 0; k < H - 1; k++) S[k] = cc::addc_cc64(S[k + 1], cc::mul_wide(a[2 * k + 1], bi));
@@ -181,7 +183,23 @@ struct Field {
 #pragma unroll
         for (int k = 1; k < H; k++) D[k] = cc::addc_cc64(D[k], cc::mul_wide(a[2 * k], bi));
         S[H - 1] = cc::pack64(cc::lo32(S[H - 1]), cc::addc(cc::hi32(S[H - 1]), 0));
+    }
+    PB_HD static void round(uint64_t *S, uint64_t *D, const uint32_t *a, uint32_t bi) {
+        shift_add_row(S, D, a, bi);
         redc_step(D, S);
+    }
+    // After the last round position 0 of B is clear: value = (B >> 32) + A  (< 2p), merged limb-wise.
+    PB_HD static Field merge(const uint64_t *A, const uint64_t *B) {
+        Field r;
+        r.l[0] = cc::add_cc(cc::lo32(A[0]), cc::hi32(B[0]));
+#pragma unroll
+        for (int k = 1; k < N - 1; k++) {
+            uint32_t x = (k & 1) ? cc::hi32(A[k >> 1]) : cc::lo32(A[k >> 1]);
+            uint32_t y = (k & 1) ? cc::lo32(B[(k + 1) >> 1]) : cc::hi32(B[k >> 1]);
+            r.l[k] = cc::addc_cc(x, y);
+        }
+        r.l[N - 1] = cc::addc(cc::hi32(A[H - 1]), 0);
+        return r;
     }
     PB_HD static Field mul_unreduced(const Field &a, const Field &b) {   // a·b/R + (< p), not brought below p: see mul_lazy
         uint64_t A[H], B[H];
@@ -197,17 +215,7 @@ struct Field {
             round(B, A, a.l, b.l[i + 1]);
         }
         round(A, B, a.l, b.l[N - 1]);
-        // the last round cleared position 0 of B: value = (B >> 32) + A  (< 2p), merged limb-wise
-        Field r;
-        r.l[0] = cc::add_cc(cc::lo32(A[0]), cc::hi32(B[0]));
-#pragma unroll
-        for (int k = 1; k < N - 1; k++) {
-            uint32_t x = (k & 1) ? cc::hi32(A[k >> 1]) : cc::lo32(A[k >> 1]);
-            uint32_t y = (k & 1) ? cc::lo32(B[(k + 1) >> 1]) : cc::hi32(B[k >> 1]);
-            r.l[k] = cc::addc_cc(x, y);
-        }
-        r.l[N - 1] = cc::addc(cc::hi32(A[H - 1]), 0);
-        return r;
+        return merge(A, B);
     }
     PB_HD static Field mul_inline(const Field &a, const Field &b) { return reduce_once(mul_unreduced(a, b)); }
 
@@ -298,22 +306,82 @@ struct Field {
             round_sqr(B, A, a, d, i + 1);
         }
         round_sqr(A, B, a, d, N - 1);
-        Field r;
-        r.l[0] = cc::add_cc(cc::lo32(A[0]), cc::hi32(B[0]));
-#pragma unroll
-        for (int k = 1; k < N - 1; k++) {
-            uint32_t u = (k & 1) ? cc::hi32(A[k >> 1]) : cc::lo32(A[k >> 1]);
-            uint32_t v = (k & 1) ? cc::lo32(B[(k + 1) >> 1]) : cc::hi32(B[k >> 1]);
-            r.l[k] = cc::addc_cc(u, v);
-        }
-        r.l[N - 1] = cc::addc(cc::hi32(A[H - 1]), 0);
-        return r;
+        return merge(A, B);
     }
     PB_HD static Field sqr_inline(const Field &x) { return reduce_once(reduce_once(sqr_unreduced(x))); }  // value < 3p
     // Lazy products for fields with ≥ 3 spare bits (Fp): BOTH operands may be lazy — a·b/R + p < (4p/R + 1)·p < 2p because
     // p/R < 1/8 — and the running value a + p < 3p (2a + p < 5p in the squaring, whose operand is pre-doubled) fits 32N bits.
     PB_HD static Field mul_lazy2(const Field &a, const Field &b) { return mul_unreduced(a, b); }
     PB_HD static Field sqr_lazy(const Field &a) { return sqr_unreduced(a); }
+
+    // ---- sum of two products, one reduction (fields with ≥ 3 spare bits: Fp) ---------------------------------------
+    // (a·b + c·d)·R⁻¹ mod p in [0, 2p) for a, b, c, d ≤ 2p: row i adds a·b_i AND c·d_i to the E / O accumulators, then runs
+    // ONE elimination step, so the two products share the N·(H + H + 1) wide multiplies of the reduction.  A difference
+    // a·b − c·d is the sum with c replaced by neg_2p(c) (which may be exactly 2p: hence ≤ 2p, not < 2p, below).
+    // Capacity, row by row.  Let U_i be the running value after row i (U_−1 = 0).  Row i forms
+    //   V_i = U_(i−1) + a·b_i + c·d_i + m_i·p ≤ U_(i−1) + (2^32 − 1)·(a + c + p),   U_i = V_i / 2^32,
+    // so by induction U_i < a + c + p and V_i < 2^32·(a + c + p) ≤ 2^32·5p < 2^32·2^384 = 2^(32(N+1)) since p < 2^381:
+    // every state of the row fits positions 0 … N of E + O·2^32.  All terms are non-negative and every carry of a chain
+    // lands at a position ≤ N, so a carry out of position N (the chains' dropped carries, the 32-bit `addc` into
+    // O[H−1]'s high half) would make the state ≥ 2^(32(N+1)) — none occurs.  Per column: the top odd column O[H−1]
+    // receives a[N−1]·b_i + c[N−1]·d_i + 2 carries < 2·2^30·2^32 + 2 (a, c < 2^382 ⇒ top limbs < 2^30), and its high half
+    // then takes the carry out of each of the two even chains (< 2^31 + 2 < 2^32); no u64 column wraps.
+    // Result: U_(N−1) = (a·b + c·d + M·p)/R with M < R, so U < (8p² + R·p)/R = 8p²/R + p < 2p because 8p < R.
+    // (Fr, one spare bit, has no room for two products: the static_assert keeps it out.)
+    PB_HD static void add_row(uint64_t *S, uint64_t *D, const uint32_t *c, uint32_t di) {   // S odd, D even: += c·d_i
+        S[0] = cc::add_cc64(S[0], cc::mul_wide(c[1], di));
+#pragma unroll
+        for (int k = 1; k < H - 1; k++) S[k] = cc::addc_cc64(S[k], cc::mul_wide(c[2 * k + 1], di));
+        S[H - 1] = cc::addc64(S[H - 1], cc::mul_wide(c[N - 1], di));
+        D[0] = cc::add_cc64(D[0], cc::mul_wide(c[0], di));
+#pragma unroll
+        for (int k = 1; k < H; k++) D[k] = cc::addc_cc64(D[k], cc::mul_wide(c[2 * k], di));
+        S[H - 1] = cc::pack64(cc::lo32(S[H - 1]), cc::addc(cc::hi32(S[H - 1]), 0));
+    }
+    PB_HD static Field mul2_sum_unreduced(const Field &a, const Field &b, const Field &c, const Field &d) {
+        static_assert(P::SPARE_BITS >= 3, "two products per row need 3 spare bits (capacity argument above)");
+        uint64_t A[H], B[H];
+#pragma unroll
+        for (int k = 0; k < H; k++) {
+            A[k] = cc::mul_wide(a.l[2 * k], b.l[0]);
+            B[k] = cc::mul_wide(a.l[2 * k + 1], b.l[0]);
+        }
+        add_row(B, A, c.l, d.l[0]);
+        redc_step(A, B);
+#pragma unroll
+        for (int i = 1; i < N - 1; i += 2) {
+            shift_add_row(A, B, a.l, b.l[i]);
+            add_row(A, B, c.l, d.l[i]);
+            redc_step(B, A);
+            shift_add_row(B, A, a.l, b.l[i + 1]);
+            add_row(B, A, c.l, d.l[i + 1]);
+            redc_step(A, B);
+        }
+        shift_add_row(A, B, a.l, b.l[N - 1]);
+        add_row(A, B, c.l, d.l[N - 1]);
+        redc_step(B, A);
+        return merge(A, B);
+    }
+    // 2p − x for x ≤ 2p, in [0, 2p]: the negated operand of a difference of products (not a lazy value: it may be 2p)
+    PB_HD Field neg_2p() const {
+        static_assert(P::SPARE_BITS >= 2, "2p must fit 32N bits");
+        Field r;
+        r.l[0] = cc::sub_cc(mod2(0), l[0]);
+#pragma unroll
+        for (int i = 1; i < N - 1; i++) r.l[i] = cc::subc_cc(mod2(i), l[i]);
+        r.l[N - 1] = cc::subc(mod2(N - 1), l[N - 1]);
+        return r;
+    }
+    PB_HD static Field mul2_sum_lazy(const Field &a, const Field &b, const Field &c, const Field &d) {   // in [0, 2p)
+        return mul2_sum_unreduced(a, b, c, d);
+    }
+    PB_HD static Field mul2_sum(const Field &a, const Field &b, const Field &c, const Field &d) {        // in [0, p)
+#if defined(PB_FIELD_NOINLINE_MUL) && defined(__CUDA_ARCH__)
+        return field_mul2_sum_noinline(a, b, c, d);
+#else
+        return reduce_once(mul2_sum_unreduced(a, b, c, d));
+#endif
+    }
     // ≡ 0 (mod p) for a lazy value: 0 or p
     PB_HD bool is_zero_lazy() const {
         uint32_t o = 0, q = 0;
@@ -387,6 +455,10 @@ __device__ __noinline__ Field<P> field_mul_noinline(Field<P> a, Field<P> b) {
 template <class P>
 __device__ __noinline__ Field<P> field_sqr_noinline(Field<P> a) {
     return Field<P>::sqr_inline(a);
+}
+template <class P>
+__device__ __noinline__ Field<P> field_mul2_sum_noinline(Field<P> a, Field<P> b, Field<P> c, Field<P> d) {
+    return Field<P>::reduce_once(Field<P>::mul2_sum_unreduced(a, b, c, d));
 }
 #endif
 

@@ -45,7 +45,7 @@ PB_HD G1Xyzz g1_dbl_affine(const G1Affine &p) {
     Fp m = xx.dbl() + xx;
     G1Xyzz r;
     r.x = m.sqr() - s.dbl();
-    r.y = m * (s - r.x) - w * p.y;
+    r.y = Fp::mul2_sum(m, s - r.x, w, p.y.neg_2p());   // m·(s − x3) − w·y, one reduction
     r.zz = v;
     r.zzz = w;
     return r;
@@ -61,7 +61,7 @@ PB_HD G1Xyzz g1_dbl(const G1Xyzz &p) {
     Fp m = xx.dbl() + xx;
     G1Xyzz r;
     r.x = m.sqr() - s.dbl();
-    r.y = m * (s - r.x) - w * p.y;
+    r.y = Fp::mul2_sum(m, s - r.x, w, p.y.neg_2p());   // m·(s − x3) − w·y, one reduction
     r.zz = v * p.zz;
     r.zzz = w * p.zzz;
     return r;
@@ -85,7 +85,7 @@ PB_HD void g1_madd(G1Xyzz &acc, const G1Affine &p) {
     Fp ppp = pp_ * pp;
     Fp q = acc.x * pp;
     Fp x3 = r.sqr() - ppp - q.dbl();
-    acc.y = r * (q - x3) - acc.y * ppp;
+    acc.y = Fp::mul2_sum(r, q - x3, acc.y.neg_2p(), ppp);   // r·(q − x3) − Y1·PPP, one reduction
     acc.x = x3;
     acc.zz = acc.zz * pp;
     acc.zzz = acc.zzz * ppp;
@@ -108,7 +108,7 @@ PB_HD void g1_madd_lazy(G1Xyzz &acc, const G1Affine &p) {
     }
     const Fp pp = Fp::sqr_lazy(pp_), ppp = Fp::mul_lazy2(pp_, pp), q = Fp::mul_lazy2(acc.x, pp);
     const Fp x3 = Fp::sub_lazy(Fp::sub_lazy(Fp::sqr_lazy(r), ppp), Fp::add_lazy(q, q));
-    acc.y = Fp::sub_lazy(Fp::mul_lazy2(r, Fp::sub_lazy(q, x3)), Fp::mul_lazy2(acc.y, ppp));
+    acc.y = Fp::mul2_sum_lazy(r, Fp::sub_lazy(q, x3), acc.y.neg_2p(), ppp);   // r·(q − x3) − Y1·PPP, one reduction
     acc.x = x3;
     acc.zz = Fp::mul_lazy2(acc.zz, pp);
     acc.zzz = Fp::mul_lazy2(acc.zzz, ppp);
@@ -140,7 +140,7 @@ PB_HD G1Xyzz g1_add(const G1Xyzz &a, const G1Xyzz &b) {
     Fp q = u1 * pp;
     G1Xyzz o;
     o.x = r.sqr() - ppp - q.dbl();
-    o.y = r * (q - o.x) - s1 * ppp;
+    o.y = Fp::mul2_sum(r, q - o.x, s1.neg_2p(), ppp);   // r·(q − x3) − S1·PPP, one reduction
     o.zz = a.zz * b.zz * pp;
     o.zzz = a.zzz * b.zzz * ppp;
     return o;

@@ -360,7 +360,7 @@ static int msm_piece(pb200_ctx *ctx, const G1Affine *bases, const uint64_t *scal
     t_sort.stop();
 
     PbTimer t_acc(ctx, "msm.accumulate");
-    // 166 registers let three CTAs share an SM; two measured faster (profiles/pipe_model_experiments_r02.txt §5), and the grid is
+    // 168 registers let three CTAs share an SM; two measured faster (profiles/pipe_model_experiments_r02.txt §5), and the grid is
     // sized in whole waves of two: 80 KiB of (unused) dynamic shared memory per CTA keeps it at two.  PB200_MSM_ACC_CTAS=3 lifts it.
     static const bool acc_three = getenv("PB200_MSM_ACC_CTAS") && atoi(getenv("PB200_MSM_ACC_CTAS")) == 3;
     const size_t acc_smem = acc_three ? 0 : 80 * 1024;
