@@ -291,7 +291,9 @@ PB200_API int pb200_prove_dev(pb200_ctx *ctx, const pb200_srs *srs, pb200_prover
  * dusk_bls12_381 (SURVEY.md §3.6, §8f-4).  No context and no GPU: the work is milliseconds and independent of n. ------- */
 /* vk_commitments: the 15 compressed commitments pb200_preprocess returns; n: padded circuit size; public inputs as for
  * pb200_prove; beta_h: the opening key's β·H ∈ G2, affine x.c0 ‖ x.c1 ‖ y.c0 ‖ y.c1 (4 × 6 u64, Montgomery).
- * Returns 0 with *accepted = 1 / 0 (a malformed proof is a rejection, not an error); PB200_ERR_ARG for bad arguments. */
+ * Returns 0 with *accepted = 1 / 0 (a malformed proof is a rejection, not an error); PB200_ERR_ARG for a null pointer, n not
+ * a power of two in [2, 2^30], a duplicate pi_gate, pi_gate[j] ≥ n or β·H not on the curve — all checked before any proof
+ * byte is looked at, so a bad argument is reported whatever the proof holds. */
 PB200_API int pb200_verify(const uint8_t vk_commitments[15 * 48], size_t n, const uint8_t *transcript_label, size_t label_len,
                            const uint8_t proof[1040], const uint32_t *pi_gate, const uint64_t *pi_mont, size_t n_pi,
                            const uint64_t beta_h[24], int *accepted);

@@ -189,6 +189,17 @@ inline HFr fr_from_bytes_wide(const uint8_t in[64]) {
     const HFr r2 = HFr::r2(), r3 = r2 * r2;
     return lo * r2 + hi * r3;
 }
+// 32 little-endian bytes → Montgomery form; false when the value is not below r (BlsScalar::from_bytes).
+inline bool fr_from_bytes_checked(const uint8_t b[32], HFr &out) {
+    HFr raw;
+    for (int i = 0; i < 4; i++) {
+        raw.l[i] = 0;
+        for (int k = 7; k >= 0; k--) raw.l[i] = (raw.l[i] << 8) | b[8 * i + k];
+    }
+    if (HFr::geq_mod(raw.l)) return false;
+    out = raw * HFr::r2();
+    return true;
+}
 // G1Affine::from(G1Projective).to_bytes(): 48 bytes, zcash compressed encoding (SURVEY.md App. A.4).
 // xyz: homogeneous projective X ‖ Y ‖ Z in Montgomery form (what pb200_msm_g1 returns).
 inline void g1_projective_to_bytes(const uint64_t xyz[18], uint8_t out[48]) {

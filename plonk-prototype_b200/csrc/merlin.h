@@ -204,4 +204,17 @@ class Transcript {
     Strobe128 strobe_;
 };
 
+// VerifierKey::seed_transcript.  vk: the 15 compressed commitments in the library's order (q_m q_l q_r q_o q_c q_4
+// q_arith q_range q_logic q_fixed_group_add q_variable_group_add σ1 σ2 σ3 σ4); upstream absorbs the variable-base selector
+// before the fixed-base one (SURVEY.md App. B.3).  The prover and both verifiers seed their transcripts here.
+inline void seed_transcript(Transcript &tr, const uint8_t vk[15 * 48], uint64_t n) {
+    const char *const label[11] = {"q_m", "q_l", "q_r", "q_o", "q_c", "q_4", "q_arith", "q_range", "q_logic", "q_variable_group_add",
+                                   "q_fixed_group_add"};
+    const int idx[11] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 10, 9};
+    for (int k = 0; k < 11; k++) tr.append_commitment(label[k], vk + 48 * idx[k]);
+    const char *const sigma[4] = {"left_sigma", "right_sigma", "out_sigma", "fourth_sigma"};
+    for (int c = 0; c < 4; c++) tr.append_commitment(sigma[c], vk + 48 * (11 + c));
+    tr.circuit_domain_sep(n);
+}
+
 }  // namespace merlin

@@ -11,6 +11,7 @@
 #pragma once
 #include <stdint.h>
 
+#include "../../include/pb200.h"
 #include "host_field.h"
 
 namespace pairing {
@@ -153,15 +154,16 @@ const uint64_t kG1y[6] = {0xbaac93d50ce72271ull, 0x8c22631a7918fd8eull, 0xdd595f
                           0x51ac582950405194ull, 0x0e1c8c3fad0059c0ull, 0x0bbc3efc5008a26aull};
 const uint64_t kFrModulus[4] = {0xffffffff00000001ull, 0x53bda402fffe5bfeull, 0x3339d80809a1d805ull, 0x73eda753299d7d48ull};
 
-// G1Affine::from_bytes (compressed): range, curve and subgroup checks as upstream.
-inline bool g1_from_bytes(const uint8_t b[48], G1A *out) {
-    if (!(b[0] & 0x80)) return false;
+// G1Affine::from_bytes (compressed): range, curve and subgroup checks as upstream.  Returns PB200_G1_* as the device
+// decoder (g1_codec.cuh) does; the identity is PB200_G1_IDENTITY with *out the point at infinity.
+inline int g1_from_bytes(const uint8_t b[48], G1A *out) {
+    if (!(b[0] & 0x80)) return PB200_G1_BAD_FLAGS;
     if (b[0] & 0x40) {
-        if (b[0] != 0xc0) return false;
+        if (b[0] != 0xc0) return PB200_G1_BAD_FLAGS;
         for (int i = 1; i < 48; i++)
-            if (b[i]) return false;
+            if (b[i]) return PB200_G1_BAD_FLAGS;
         *out = {HFp::zero(), HFp::zero(), true};
-        return true;
+        return PB200_G1_IDENTITY;
     }
     HFp raw;
     for (int i = 0; i < 6; i++) {
@@ -172,13 +174,13 @@ inline bool g1_from_bytes(const uint8_t b[48], G1A *out) {
             raw.l[i] = (raw.l[i] << 8) | byte;
         }
     }
-    if (HFp::geq_mod(raw.l)) return false;
+    if (HFp::geq_mod(raw.l)) return PB200_G1_X_RANGE;
     const HFp x = raw * HFp::r2();
     const HFp rhs = x.sqr() * x + HFp::from_u64(4);
     static const uint64_t kSqrtExp[6] = {0xee7fbfffffffeaabull, 0x07aaffffac54ffffull, 0xd9cc34a83dac3d89ull,
                                          0xd91dd2e13ce144afull, 0x92c6e9ed90d2eb35ull, 0x0680447a8e5ff9a6ull};  // (p + 1)/4
     HFp y = rhs.pow(kSqrtExp, 6);
-    if (y.sqr() != rhs) return false;
+    if (y.sqr() != rhs) return PB200_G1_NOT_ON_CURVE;
     // choose the root the flag asks for: larger ⇔ 2y ≥ p
     const HFp yc = y.from_mont();
     uint64_t d[6], c = 0;
@@ -196,7 +198,7 @@ inline bool g1_from_bytes(const uint8_t b[48], G1A *out) {
         acc = g1_double(acc);
         if ((kFrModulus[i >> 6] >> (i & 63)) & 1) acc = g1_add(acc, p);
     }
-    return acc.is_identity();
+    return acc.is_identity() ? PB200_G1_OK : PB200_G1_NOT_IN_SUBGROUP;
 }
 
 // ------------------------------------------------------------------------------------------------ G2 (affine) / pairing

@@ -33,10 +33,6 @@ namespace {
 
 constexpr int kSel = 11;  // q_m q_l q_r q_o q_c q_4 q_arith q_range q_logic q_fixed_group_add q_variable_group_add
 enum { Q_M, Q_L, Q_R, Q_O, Q_C, Q_4, Q_ARITH, Q_RANGE, Q_LOGIC, Q_FIXED, Q_VAR };
-const char *const kSelLabel[kSel] = {"q_m", "q_l", "q_r", "q_o", "q_c", "q_4", "q_arith", "q_range", "q_logic",
-                                     "q_fixed_group_add", "q_variable_group_add"};
-// VerifierKey::seed_transcript absorbs the variable-base selector before the fixed-base one (SURVEY.md App. B.3).
-const int kSeedOrder[kSel] = {Q_M, Q_L, Q_R, Q_O, Q_C, Q_4, Q_ARITH, Q_RANGE, Q_LOGIC, Q_VAR, Q_FIXED};
 
 inline Fr to_dev(const HFr &h) {  // same memory image: 4 × u64 LE = 8 × u32 LE
     Fr r;
@@ -765,10 +761,7 @@ extern "C" int pb200_preprocess_sharded(pb200_ctx *ctx, const pb200_srs *srs, co
 
     // Transcript::new(label) seeded with the verifier key
     pk->seeded = new merlin::Transcript(transcript_label, label_len);
-    for (int k = 0; k < kSel; k++) pk->seeded->append_commitment(kSelLabel[kSeedOrder[k]], vk + 48 * kSeedOrder[k]);
-    const char *const sig_label[4] = {"left_sigma", "right_sigma", "out_sigma", "fourth_sigma"};
-    for (int c = 0; c < 4; c++) pk->seeded->append_commitment(sig_label[c], vk + 48 * (kSel + c));
-    pk->seeded->circuit_domain_sep(n);
+    merlin::seed_transcript(*pk->seeded, vk, n);
     if (vk_commitments) memcpy(vk_commitments, vk, sizeof(pk->vk_bytes));
     *out = pk;
     return 0;

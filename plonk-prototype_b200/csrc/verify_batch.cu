@@ -16,7 +16,6 @@
 //   3. (host) D = Merlin("pb200 verify_batch") over the seed, n, K and every digest;
 //   4. verify_weight_kernel, one thread per proof: ρ_k, the two MSM scalar vectors, placeholder bases for identity slots;
 //   5. verify_colsum_kernel: shared-base scalars over a proof range; then the MSMs (msm.cu) and the pairing (host).
-#include <algorithm>
 #include <chrono>
 #include <cstring>
 #include <vector>
@@ -26,7 +25,6 @@
 #include "verify_batch.cuh"
 
 using hostf::HFp;
-using hostf::HFr;
 
 namespace {
 
@@ -35,13 +33,13 @@ constexpr int kPts = vb::kProofPoints, kSh = vb::kShared;
 // One thread per proof.  Writes the proof's C-side coefficients (kPts), shared-base coefficients (kSh), u_k, its digest
 // and its verdict; a rejected proof writes its verdict only.
 __global__ void __launch_bounds__(128) verify_prepare_kernel(const merlin::Transcript seed, const uint8_t *__restrict__ proofs,
-                                                             const uint8_t *__restrict__ pt_status, const vb::Consts k,
+                                                             const uint8_t *__restrict__ pt_status, const vb::Consts<Fr> k,
                                                              const Fr *__restrict__ wg, const Fr *__restrict__ pi, uint32_t K,
                                                              Fr *__restrict__ coef, Fr *__restrict__ ecoef, Fr *__restrict__ u_out,
                                                              uint8_t *__restrict__ digest, uint8_t *__restrict__ verdict) {
     const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= K) return;
-    vb::ProofOut o;
+    vb::ProofOut<Fr> o;
     const int st = vb::prepare_one(seed, proofs + 1040 * (size_t)p, pt_status + kPts * (size_t)p, k, wg, pi + (size_t)k.n_pi * p, o);
     verdict[p] = (uint8_t)st;
     if (st != vb::OK) {
@@ -219,20 +217,6 @@ int bisect(Checker &ck, const std::vector<uint32_t> &surv_prefix, const std::vec
     return bisect(ck, surv_prefix, alive, mid, hi, left_pass, accepted);
 }
 
-HFr host_omega(size_t n) {
-    uint32_t log_n = 0;
-    while (((size_t)1 << log_n) < n) log_n++;
-    const uint64_t root32[4] = {0xb9b58d8c5f0e466aull, 0x5b1b4c801819d7ecull, 0x0af53ae352a31e64ull, 0x5bf3adda19e9b27bull};
-    HFr omega = HFr::load(root32);
-    for (uint32_t k = 0; k < 32 - log_n; k++) omega = omega.sqr();
-    return omega;
-}
-Fr to_dev(const HFr &a) {
-    Fr r;
-    memcpy(r.l, a.l, 32);
-    return r;
-}
-
 int run(pb200_ctx *ctx, Bufs &b, const uint8_t *vk_commitments, size_t n, const uint8_t *label, size_t label_len, const uint8_t *proofs,
         size_t K, const uint32_t *pi_gate, const uint64_t *pi_mont, size_t n_pi, const pairing::G2A &bh, const uint8_t seed[32],
         uint8_t *accepted, int *all_accepted) {
@@ -266,27 +250,9 @@ int run(pb200_ctx *ctx, Bufs &b, const uint8_t *vk_commitments, size_t n, const 
 
         // 2. per-proof derivation
         merlin::Transcript tr(label, label_len);
-        {
-            enum { Q_M, Q_L, Q_R, Q_O, Q_C, Q_4, Q_ARITH, Q_RANGE, Q_LOGIC, Q_FIXED, Q_VAR, S1 };
-            const char *const lab[11] = {"q_m", "q_l", "q_r", "q_o", "q_c", "q_4", "q_arith", "q_range", "q_logic", "q_variable_group_add",
-                                         "q_fixed_group_add"};
-            const int idx[11] = {Q_M, Q_L, Q_R, Q_O, Q_C, Q_4, Q_ARITH, Q_RANGE, Q_LOGIC, Q_VAR, Q_FIXED};
-            for (int q = 0; q < 11; q++) tr.append_commitment(lab[q], vk_commitments + 48 * idx[q]);
-            const char *const sl[4] = {"left_sigma", "right_sigma", "out_sigma", "fourth_sigma"};
-            for (int c = 0; c < 4; c++) tr.append_commitment(sl[c], vk_commitments + 48 * (S1 + c));
-            tr.circuit_domain_sep(n);
-        }
-        vb::Consts kc;
-        const HFr omega = host_omega(n), n_fr = HFr::from_u64(n);
-        kc.n = n;
-        kc.n_pi = (uint32_t)n_pi;
-        kc.vk_identity = vk_identity;
-        kc.omega = to_dev(omega);
-        kc.n_fr = to_dev(n_fr);
-        kc.n_inv = to_dev(n_fr.inv());
-        kc.edwards_d = to_dev((HFr::from_u64(10240) * HFr::from_u64(10241).inv()).neg());
-        std::vector<uint64_t> wg(4 * (n_pi ? n_pi : 1));
-        for (size_t j = 0; j < n_pi; j++) omega.pow_u64(pi_gate[j]).store(&wg[4 * j]);
+        merlin::seed_transcript(tr, vk_commitments, n);
+        std::vector<Fr> wg;
+        const vb::Consts<Fr> kc = vb::make_consts(n, pi_gate, n_pi, vk_identity, wg);
         if (n_pi) {
             PB_CUDA(ctx, cudaMemcpyAsync(b.wg, wg.data(), 32 * n_pi, cudaMemcpyHostToDevice, st));
             PB_CUDA(ctx, cudaMemcpyAsync(b.pi, pi_mont, 32 * n_pi * K, cudaMemcpyHostToDevice, st));
@@ -354,16 +320,9 @@ extern "C" int pb200_verify_batch(pb200_ctx *ctx, const uint8_t vk_commitments[1
     PB_ARG(ctx, vk_commitments && proofs && beta_h && seed && accepted && all_accepted);
     PB_ARG(ctx, !n_pi || (pi_gate && pi_mont));
     PB_ARG(ctx, transcript_label || !label_len);
-    PB_ARG(ctx, n >= 2 && !(n & (n - 1)) && n <= ((size_t)1 << 30));
     PB_ARG(ctx, n_proofs >= 1 && n_proofs <= ((size_t)1 << 20));
-    if (n_pi > 1) {
-        std::vector<uint32_t> sorted(pi_gate, pi_gate + n_pi);
-        std::sort(sorted.begin(), sorted.end());
-        PB_ARG(ctx, std::adjacent_find(sorted.begin(), sorted.end()) == sorted.end());
-    }
-    for (size_t j = 0; j < n_pi; j++) PB_ARG(ctx, pi_gate[j] < n);
-    const pairing::G2A bh = {{HFp::load(beta_h), HFp::load(beta_h + 6)}, {HFp::load(beta_h + 12), HFp::load(beta_h + 18)}, false};
-    PB_ARG(ctx, pairing::g2_on_curve(bh));
+    pairing::G2A bh;
+    PB_ARG(ctx, vb::args_ok(n, pi_gate, n_pi, beta_h, &bh));
     memset(accepted, 0, n_proofs);
     *all_accepted = 0;
     PB_CUDA(ctx, cudaSetDevice(ctx->device));

@@ -1,9 +1,9 @@
 // widgets.h — the logic, fixed-base and variable-base widget identities of dusk-plonk 0.8
 // (proof_system::widget::{logic, ecc::scalar_mul::fixed_base, ecc::curve_addition}; crate pinned at
 // /root/reference/Cargo.toml:19, driven by the reference at /root/reference/src/zk/gadgets.rs:34-40 and circuits.rs:64).
-// One generic definition over the field type F, instantiated three ways: Fr on the device (quotient_kernel, one coset
-// point per thread), hostf::HFr in the prover's linearisation (plonk.cu) and in the verifier (verify.cu) — as upstream
-// shares one formula between `compute_quotient_i` and `compute_linearisation`.
+// One generic definition over the field type F: Fr on the device (quotient_kernel, one coset point per thread, and the
+// batched verifier), hostf::HFr in the prover's linearisation (plonk.cu) and in pb200_verify (both verifiers through
+// verify_batch.cuh) — as upstream shares one formula between `compute_quotient_i` and `compute_linearisation`.
 // F needs + − * and F::one().  Formulas restated from memory of the crate (UPSTREAM_ASSUMPTIONS.md §widgets); the logic
 // polynomial and the JubJub constant are additionally pinned by mathematics (tests/test_widgets_cpu.py).
 #pragma once

@@ -1,22 +1,13 @@
 // Host-emulation harness for the batched verifier's per-proof derivation (csrc/verify_batch.cuh, the code
 // verify_prepare_kernel and verify_weight_kernel run), compiled for the CPU with the carry-flag primitives emulated
-// (PB200_HOST_EMU), behind a C ABI for pytest.  The host-side set-up mirrors pb200_verify_batch (csrc/verify_batch.cu).
+// (PB200_HOST_EMU), behind a C ABI for pytest.  The host-side set-up is pb200_verify_batch's (merlin::seed_transcript,
+// vb::make_consts), called here as there.
 #define PB200_HOST_EMU 1
 #include "../../plonk-prototype_b200/csrc/g1_codec.cuh"
 #include "../../plonk-prototype_b200/csrc/verify_batch.cuh"
 #include <cstddef>
 #include <cstring>
 #include <vector>
-
-using hostf::HFr;
-
-namespace {
-Fr to_fr(const HFr &a) {
-    Fr r;
-    memcpy(r.l, a.l, 32);
-    return r;
-}
-}  // namespace
 
 extern "C" {
 // One proof through vb::prepare_one.  Returns -1 for a malformed verifier key, else the verdict (vb::OK = 0 …).  For OK:
@@ -37,33 +28,11 @@ int emu_verify_prepare(const uint8_t *label, size_t label_len, const uint8_t *vk
         pt_status[i] = (uint8_t)g1_decode_checked(proof + 48 * i, p);
     }
     merlin::Transcript tr(label, label_len);
-    const char *const lab[11] = {"q_m", "q_l", "q_r", "q_o", "q_c", "q_4", "q_arith", "q_range", "q_logic", "q_variable_group_add",
-                                 "q_fixed_group_add"};
-    const int idx[11] = {0, 1, 2, 3, 4, 5, 6, 7, 8, 10, 9};
-    for (int q = 0; q < 11; q++) tr.append_commitment(lab[q], vk + 48 * idx[q]);
-    const char *const sl[4] = {"left_sigma", "right_sigma", "out_sigma", "fourth_sigma"};
-    for (int c = 0; c < 4; c++) tr.append_commitment(sl[c], vk + 48 * (11 + c));
-    tr.circuit_domain_sep(n);
-    uint32_t log_n = 0;
-    while ((1ull << log_n) < n) log_n++;
-    const uint64_t root32[4] = {0xb9b58d8c5f0e466aull, 0x5b1b4c801819d7ecull, 0x0af53ae352a31e64ull, 0x5bf3adda19e9b27bull};
-    HFr omega = HFr::load(root32);
-    for (uint32_t k = 0; k < 32 - log_n; k++) omega = omega.sqr();
-    vb::Consts kc;
-    const HFr n_fr = HFr::from_u64(n);
-    kc.n = n;
-    kc.n_pi = (uint32_t)n_pi;
-    kc.vk_identity = vk_identity;
-    kc.omega = to_fr(omega);
-    kc.n_fr = to_fr(n_fr);
-    kc.n_inv = to_fr(n_fr.inv());
-    kc.edwards_d = to_fr((HFr::from_u64(10240) * HFr::from_u64(10241).inv()).neg());
-    std::vector<Fr> wg(n_pi + 1), pi(n_pi + 1);
-    for (size_t j = 0; j < n_pi; j++) {
-        wg[j] = to_fr(omega.pow_u64(pi_gate[j]));
-        memcpy(pi[j].l, pi_mont + 4 * j, 32);
-    }
-    vb::ProofOut o;
+    merlin::seed_transcript(tr, vk, n);
+    std::vector<Fr> wg, pi(n_pi);
+    const vb::Consts<Fr> kc = vb::make_consts(n, pi_gate, n_pi, vk_identity, wg);
+    for (size_t j = 0; j < n_pi; j++) memcpy(pi[j].l, pi_mont + 4 * j, 32);
+    vb::ProofOut<Fr> o;
     const int st = vb::prepare_one(tr, proof, pt_status, kc, wg.data(), pi.data(), o);
     if (st != vb::OK) return st;
     for (int i = 0; i < 11; i++) memcpy(coef + 4 * i, o.coef[i].l, 32);
